@@ -1,7 +1,7 @@
 """Headline benchmark: audio-seconds/s of prefill (and TTFT p50) for Ultravox-v0.5-shaped random-init weights
 (Whisper-large-v3 encoder + Llama-3.1-8B), synthetic 30 s / 16 kHz clips, batch 1 per GPU, data-parallel replicas.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--preset v0_5_8b] [--secs 30]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--preset v0_5_8b] [--secs 30] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one full pass of the hot path over one clip: waveform -> log-mel -> encoder -> projector -> splice -> Llama
@@ -22,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "audio-sec/s prefill (Llama-3.1-8B, 30s clip) at 1/2/4/8 B200; TTFT p50"
 UNIT = "audio-sec/s"
@@ -45,7 +46,24 @@ def parse():
     ap.add_argument("--ttft-iters", type=int, default=200, help="end-to-end iterations behind TTFT p50 / p90 (>= --steps)")
     ap.add_argument("--cpu-threads", type=int, default=0, help="host threads of the CPU arm (0 = sweep and keep the fastest)")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="wall-clock budget of the CPU arm's timed steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0: last-position logits, greedy token) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """One float32 / float64 .npy per output, so that two builds run with the same arguments can be compared array by array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu()
+        a = a.float() if a.is_floating_point() else a.double()     # integer outputs (token ids < 2**53) are exact in float64
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
 
 
 def workload(cfg, secs):
@@ -596,6 +614,7 @@ def main():
         eng.run()
     e1.record()
     barrier()
+    last_step = {"logits": eng.logits.clone(), "token": eng.token.clone()}    # the later passes overwrite the engine's buffers
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -696,6 +715,8 @@ def main():
                 line["token_check"] = bool(tokens_ok and check["ok"])
             except Exception as e:      # e.g. host RAM too small for the fp32 copy: keep the headline, say what happened
                 line["cpu_baseline"] = {"error": repr(e)[:300]}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
